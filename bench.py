@@ -20,6 +20,9 @@ ranks.  `stage_ms` / `roofline` come from a serial pass on ONE context whose str
 the per-kernel CUDA events there time exactly one kernel each.  Inputs exceed L2 (126 MB) in every config.
 Parity: every block / digest / fragment table of the timed batch is compared with the reference (oracle/_ref, run once
 on all host cores, outside the timed region) -- config.parity says how many matched.
+--dump-outputs DIR: after the timed steps, what the last timed step returned is written as DIR/<name>.npy (float32 /
+float64, at most 64 MB): block offsets and lengths, the SHA-256 of every block and a fixed sample of whole blocks; c4
+the fragment tables and digests.  The inputs depend on the arguments only, so two builds can be compared file by file.
 """
 import argparse
 import hashlib
@@ -35,6 +38,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the tree may be read-only; nothing is written into it
 
 UNIT = 65536
 MB = 1e6
@@ -46,6 +50,8 @@ METRICS = {
 }
 # state bytes read+written per coded bit (SURVEY.md section 8d): S = sum over the model's components
 S_BYTES = {"3": 28, "4": 157, "5": 573}
+DUMP_CAP = 64 << 20       # --dump-outputs: bytes written at most
+DUMP_SAMPLE = 128         # --dump-outputs: blocks of a batch written whole (a seeded choice; all by SHA-256)
 
 
 def load_corpus():
@@ -94,6 +100,28 @@ class ClockSampler(threading.Thread):
         reasons = [n for k, n in enumerate(names) if any(len(r) > 2 + k and r[2 + k] == "Active" for r in self.rows)]
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None, "reasons": reasons,
                 "samples": len(self.rows)}
+
+
+def block_outputs(data, ooff, olen, prefix=""):
+    """What a caller of a batch entry point receives -- blocks data[ooff[i]:ooff[i]+olen[i]], their offsets and lengths --
+    as float arrays for --dump-outputs: every block by its SHA-256, a seeded sample of DUMP_SAMPLE blocks byte for byte."""
+    n = len(olen)
+    blocks = [data[int(ooff[i]): int(ooff[i]) + int(olen[i])] for i in range(n)]
+    pick = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_SAMPLE), replace=False))
+    sha = np.frombuffer(b"".join(hashlib.sha256(b).digest() for b in blocks), dtype=np.uint8).reshape(n, 32)
+    return {prefix + "offsets": np.asarray(ooff, dtype=np.float64), prefix + "lengths": np.asarray(olen, dtype=np.float64),
+            prefix + "sha256": sha.astype(np.float32), prefix + "sample_index": pick.astype(np.float64),
+            prefix + "sample_bytes": np.concatenate([blocks[i] for i in pick] + [np.zeros(0, np.uint8)]).astype(np.float32)}
+
+
+def dump_outputs(directory, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_CAP:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte cap (a smaller workload dumps less)" % (total, DUMP_CAP))
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), name
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 # ---- synthetic workloads (same bytes for both arms) ------------------------------------------------------------
@@ -306,6 +334,7 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--inflight", type=int, default=4,
                     help="c2: batches in flight (zq_pipe lanes): the next step's copies/kernels fill the tail of the current one")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -367,9 +396,10 @@ def main():
     peak, peak_src = load_peaks()
     ref = None if args.no_parity and args.no_cpu_baseline else ref_lib()
     line = None
+    outputs = {}
 
     if cfg == "c4":
-        line = run_c4(args, zq, corpus, ctx, zd, ref, rank, world, local, dist, torch, bracket, sync_all, peak, peak_src)
+        line = run_c4(args, zq, corpus, ctx, zd, ref, rank, world, local, dist, torch, bracket, sync_all, peak, peak_src, outputs)
     else:
         arena_np, offs, lens = make_units(corpus, cfg, rank, args)
         U = len(offs)
@@ -414,6 +444,7 @@ def main():
                 r_ = pipe.wait(t)
                 if world > 1 and not device:
                     exchange(r_[1])
+            state["last"] = ((steps - 1) % depth, r_)      # the last step's output buffer, (offsets, lengths)
             torch.cuda.synchronize()
             e1.record(stream)
             sync_all()
@@ -426,6 +457,9 @@ def main():
             piped(max(args.warmup, depth), True)
             sampler.start()
             ms_dev, launches = piped(args.steps, True)
+            if args.dump_outputs:
+                k, (ooff, olen) = state["last"]
+                outputs.update(block_outputs(d_outs[k][:int((ooff + olen).max())].cpu().numpy(), ooff, olen))
             piped(max(args.warmup, depth), False)
             ms_e2e, _ = piped(args.steps, False)
             d2h_extra = h2d_extra = 0
@@ -438,6 +472,9 @@ def main():
             l0 = ctx.launch_count()
             ms_dev = bracket(step_device, args.steps)
             launches = ctx.launch_count() - l0
+            if args.dump_outputs:
+                ooff, olen = state["dev"]
+                outputs.update(block_outputs(d_outs[0][:int((ooff + olen).max())].cpu().numpy(), ooff, olen))
             for _ in range(max(1, args.warmup - 1)):
                 step_host()
             ms_e2e = bracket(step_host, args.steps)
@@ -452,6 +489,8 @@ def main():
                 l0 = ctx.launch_count()
                 ms_dec = bracket(step_dec, args.steps)
                 launches += ctx.launch_count() - l0
+                if args.dump_outputs:
+                    outputs.update(block_outputs(*dstate["dec"], prefix="decoded_"))
                 ms_dev += ms_dec
                 ms_e2e += ms_dec
                 h2d_extra, d2h_extra = int(clen.sum()), nbytes
@@ -547,6 +586,8 @@ def main():
         if pipe is not None:
             pipe.close()
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     zd.close()
     ctx.close()
@@ -555,7 +596,7 @@ def main():
     return 0
 
 
-def run_c4(args, zq, corpus, ctx, zd, ref, rank, world, local, dist, torch, bracket, sync_all, peak, peak_src):
+def run_c4(args, zq, corpus, ctx, zd, ref, rank, world, local, dist, torch, bracket, sync_all, peak, peak_src, outputs):
     """Fragmenter + fragment SHA-1 + per-file BLAKE3 over this rank's share of the image; digests all-gathered."""
     sizes, kinds, srcs = make_image(corpus, int(args.c4_gb * 1e9))
     # files dealt to the ranks longest first (LPT): every rank computes the same assignment
@@ -587,6 +628,10 @@ def run_c4(args, zq, corpus, ctx, zd, ref, rank, world, local, dist, torch, brac
     sampler.stop_flag = True
     sampler.join(timeout=3)
     fl, fh, fs, first = res["frag"]
+    if args.dump_outputs:
+        outputs.update({"fragment_lengths": fl.astype(np.float64), "fragment_hits": fh.astype(np.float64),
+                        "fragment_sha1": fs.astype(np.float32), "file_first_fragment": first.astype(np.float64),
+                        "file_blake3": np.asarray(res["b3"]).astype(np.float32)})
     # dedup key exchange: 20-byte digests of every rank's fragments -> global unique count (the index the archiver keeps)
     nfrag = len(fl)
     torch.cuda.synchronize()

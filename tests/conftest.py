@@ -44,10 +44,16 @@ def oracle():
 
 @pytest.fixture(scope="session")
 def ref():
-    """oracle/_ref/libzpaqref.so -- the reference itself, compiled from /root/reference (checker)."""
-    _ensure_built()
+    """The reference's answers (checker): recorded under tests/golden/ref/.  With ZQ_RECORD_REF=<dir> set, the reference
+    itself (oracle/_ref/libzpaqref.so), every answer written to <dir>/<test module>.json at the end of the session."""
     import oracle_bindings
+    out = os.environ.get("ZQ_RECORD_REF")
+    if not out:
+        yield oracle_bindings.GoldenRef()
+        return
+    _ensure_built()
     r = oracle_bindings.load_ref()
-    if r is None:
-        pytest.skip("oracle/_ref/libzpaqref.so not available")
-    return r
+    assert r is not None, "ZQ_RECORD_REF needs the reference: oracle/_ref/libzpaqref.so is not built"
+    rec = oracle_bindings.RecordingRef(r)
+    yield rec
+    rec.save(out)

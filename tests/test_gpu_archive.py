@@ -1,10 +1,8 @@
 """Archive-level parity: the data ("d") and fragment-table ("h") blocks of an archive written by the REFERENCE's
-own command line (`zpaqfranz a`, run through oracle/_ref) are reproduced byte for byte by zq_add_files -- the
-device fragmenter + SHA-1 + order-1 tables, the host dedup / type heuristics / new-block rule, and the device
-block compressor.  (SURVEY §8 a15-a17, §8f rank 2.)"""
+own command line (`zpaqfranz a`, recorded by oracle_bindings.Ref.archive_d_h) are reproduced byte for byte by
+zq_add_files -- the device fragmenter + SHA-1 + order-1 tables, the host dedup / type heuristics / new-block rule, and
+the device block compressor.  (SURVEY §8 a15-a17, §8f rank 2.)"""
 import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -13,52 +11,6 @@ import zpaqfranz_b200 as zqmod
 from zpaqfranz_b200 import corpus
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-TAG = bytes([0x37, 0x6b, 0x53, 0x74, 0xa0, 0x31, 0x83, 0xd3, 0x8c, 0xb2, 0x28, 0xb0, 0xd3]) + b"zPQ"
-
-
-def reference_archive(src_dir, archive, *flags):
-    """Run the reference's main() on `a <archive> <src_dir> flags...` in a child process."""
-    code = ("import ctypes as C, sys\n"
-            "lib = C.CDLL(%r)\n"
-            "a = [x.encode() for x in sys.argv[1:]]\n"
-            "arr = (C.c_char_p * len(a))(*a)\n"
-            "lib.zref_main.restype = C.c_int\n"
-            "sys.exit(lib.zref_main(len(a), arr))\n") % os.path.join(ROOT, "oracle", "_ref", "libzpaqref.so")
-    r = subprocess.run([sys.executable, "-c", code, "zpaqfranz", "a", str(archive), str(src_dir)] + list(flags),
-                       capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    return open(archive, "rb").read()
-
-
-def split_blocks(blob):
-    """[(kind, name, block bytes)] of a journaling archive: kind is the letter after the 14-digit date."""
-    starts = []
-    p = blob.find(TAG)
-    while p >= 0:
-        starts.append(p)
-        p = blob.find(TAG, p + 16)
-    out = []
-    for i, s in enumerate(starts):
-        e = starts[i + 1] if i + 1 < len(starts) else len(blob)
-        b = blob[s:e]
-        q = 18
-        q += 2 + b[q] + 256 * b[q + 1]
-        assert b[q] == 1
-        name = b[q + 1: b.index(b"\0", q + 1)].decode()
-        assert name.startswith("jDC")
-        out.append((name[17], name, b))
-    return out
-
-
-def make_tree(root, spec):
-    for rel, data in spec.items():
-        p = os.path.join(root, rel)
-        os.makedirs(os.path.dirname(p), exist_ok=True)
-        with open(p, "wb") as f:
-            f.write(data)
-
-
 TREES = {
     "small_mixed": {
         "a.txt": corpus.text_unit(1, 300000), "b.bin": corpus.random_unit(2, 100000), "sub/c.txt": corpus.text_unit(1, 300000),
@@ -74,19 +26,14 @@ TREES = {
 @pytest.mark.parametrize("tree,flags", [("small_mixed", ["-m2"]), ("small_mixed", ["-m1"]), ("small_mixed", ["-m3"]),
                                         ("small_mixed", ["-m20", "-fragment", "4"]), ("many_blocks", ["-m10"]),
                                         ("many_blocks", ["-m21"]), ("small_mixed", ["-m4"])])
-def test_d_and_h_blocks_match_the_reference_archiver(ctx, tmp_path, tree, flags):
-    src = tmp_path / "src"
-    make_tree(str(src), TREES[tree])
-    blob = reference_archive(src, tmp_path / "t.zpaq", *flags)
-    blocks = split_blocks(blob)
-    date14 = blocks[0][1][3:17]
-    want_d = b"".join(b for k, _, b in blocks if k == "d")
-    want_h = b"".join(b for k, _, b in blocks if k == "h")
+def test_d_and_h_blocks_match_the_reference_archiver(ctx, ref, tree, flags):
+    src = "/archived/src"      # any common prefix: the order below depends on the paths below it only
+    date14, nblocks, want_d, want_h = ref.archive_d_h(TREES[tree], flags)
     assert want_d and want_h
     # files in the reference's order: sort key, then full path (Z:121735-121754, compareFilename Z:63575)
     files = []
     for rel, data in TREES[tree].items():
-        path = os.path.join(str(src), rel)
+        path = os.path.join(src, rel)
         files.append((zqmod.file_sort_key(path, len(data)), path, data))
     files.sort(key=lambda t: (t[0], t[1]))
     lens = np.array([len(f[2]) for f in files], dtype=np.uint64)
@@ -95,11 +42,11 @@ def test_d_and_h_blocks_match_the_reference_archiver(ctx, tmp_path, tree, flags)
     method = flags[0][2:]
     fragment = int(flags[flags.index("-fragment") + 1]) if "-fragment" in flags else 6
     got = ctx.add_files(arena, offs, lens, method=method, fragment=fragment, date14=date14)
-    assert got["nblocks"] == sum(1 for k, _, _ in blocks if k == "d")
+    assert got["nblocks"] == nblocks
     assert got["d"] == want_d
     assert got["h"] == want_h
     # every file is covered by its fragment list, duplicates share ids
-    names = [os.path.relpath(f[1], str(src)) for f in files]
+    names = [os.path.relpath(f[1], src) for f in files]
     ids = dict(zip(names, got["file_frags"]))
     if tree == "small_mixed":
         assert ids["a.txt"] == ids["sub/c.txt"]

@@ -17,10 +17,21 @@ def _pack(blobs):
     return np.frombuffer(b"".join(blobs) + b"\0", dtype=np.uint8), offs, lens
 
 
+def _reference_blocks(ctx, ref, units, method, filename, comment, dosha1=True):
+    """The blocks the reference writes for `units`: made by the device compressor, each one checked equal to the
+    reference's (whose recorded answer for a large block is its digest, not its bytes)."""
+    arena, offs, lens = _pack(units)
+    out, ooff, olen = ctx.compress_blocks(arena, offs, lens, method=method, filename=filename, comment=comment, dosha1=dosha1)
+    blocks = [out[int(ooff[i]): int(ooff[i]) + int(olen[i])].tobytes() for i in range(len(units))]
+    for i, u in enumerate(units):
+        assert blocks[i] == ref.compress_block(u, method, filename, comment, dosha1=dosha1), (method, i, len(u))
+    return blocks
+
+
 @pytest.mark.parametrize("method", ["0", "1", "2", "3", "36,200,1", "4", "46,200,1", "1,128,2", "3,200,3", "x0,4", "x0,7ci1",
                                      "x0,2,12,0,7,21,1c0,0,511i2", "x0,0c0,0,255i2,13m8,24s", "x0,6,12,0,7,21,1c0,0,511i2"])
 def test_decode_reference_blocks(ctx, ref, method):
-    blocks = [ref.compress_block(u, method, "name", "jDC\x01") for u in UNITS]
+    blocks = _reference_blocks(ctx, ref, UNITS, method, "name", "jDC\x01")
     arena, offs, lens = _pack(blocks)
     out, ooff, olen = ctx.decompress_blocks(arena, offs, lens)
     for i, u in enumerate(UNITS):
@@ -31,7 +42,7 @@ def test_decode_reference_blocks(ctx, ref, method):
 def test_decode_m5_and_no_checksum(ctx, ref):
     units = UNITS[:7]
     for method, sha in (("5", True), ("2", False), ("4", False)):
-        blocks = [ref.compress_block(u, method, "", "c", dosha1=sha) for u in units]
+        blocks = _reference_blocks(ctx, ref, units, method, "", "c", dosha1=sha)
         arena, offs, lens = _pack(blocks)
         out, ooff, olen = ctx.decompress_blocks(arena, offs, lens, expect_len=[len(u) for u in units])
         for i, u in enumerate(units):
@@ -50,7 +61,7 @@ def test_gpu_round_trip(ctx):
 
 
 def test_corruption_is_detected(ctx, ref, zq):
-    blk = bytearray(ref.compress_block(corpus.text_unit(1, 20000), "3", "", "jDC\x01"))
+    blk = bytearray(_reference_blocks(ctx, ref, [corpus.text_unit(1, 20000)], "3", "", "jDC\x01")[0])
     blk[len(blk) // 2] ^= 0x5A
     arena, offs, lens = _pack([bytes(blk)])
     with pytest.raises(zq.ZqError):
